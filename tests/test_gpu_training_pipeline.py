@@ -43,7 +43,7 @@ def test_training_pipeline_runs_and_writes_reference_artifacts(tmp_path, agent):
     assert (per_step > 0).all() and (per_step <= 1.0 + 1e-9).all()
 
 
-def test_sac_training_beats_the_random_policy():
+def test_sac_training_beats_the_random_policy(tmp_path):
     """Evidence that the driver trains (VERDICT r1 missing #5; the reference claims a rising reward curve,
     problem-04-sac-gru/README.md:461-464).  8 servers, four fast (speed 2) and four slow (speed 1): weights
     proportional to speed even out the flow durations (Jain 0.92), equal weights give 0.86, the random policy --
@@ -56,7 +56,7 @@ def test_sac_training_beats_the_random_policy():
     speeds = [2.0, 2.0, 2.0, 2.0, 1.0, 1.0, 1.0, 1.0]
     cfg = dict(server_speeds=speeds, rates=[24.0], seed=1, updates_per_round=100, batch_size=256)
     torch.manual_seed(0); np.random.seed(0); random.seed(0)
-    tp = TrainingPipeline('sac-gru', num_servers=8, num_agents=1, trace_dir='/nonexistent', checkpoint_dir='/tmp/mlb_learn_ck',
+    tp = TrainingPipeline('sac-gru', num_servers=8, num_agents=1, trace_dir=str(tmp_path / 'no_traces'), checkpoint_dir=str(tmp_path),
                           config=cfg, num_envs=16, verbose=False)
     E = tp.num_envs
 
