@@ -51,10 +51,11 @@ struct mlb_env {
     size_t action_bytes = 0;
     uint8_t* d_mask = nullptr;
     size_t ev_smem = 0, ft_smem = 0, pr_smem = 0;   // dynamic shared memory of the event / feature / pair kernel
-    bool use_pair = false;             // pair_kernel applies (128-slot reservoirs, feature cache on)
-    int pair_wpe_small = 4;            // warps per (env, agent) in pair_kernel for launches of <= 8192 (env, agent) pairs
-    // small launches: pair_kernel<.,1> runs BESIDE pair_kernel<.,0> (disjoint reservoirs) on this stream -- under a
-    // stream capture a parallel branch of the graph; at those sizes each launch is one warp's latency chain
+    const void *ev_fn = nullptr, *ft_fn = nullptr, *pr_fn[2] = {nullptr, nullptr};   // kernel instantiations of this config
+    bool use_pair = false;             // pair_kernel applies (128-slot reservoir stride, feature cache on)
+    // small launches (<= 8192 (env, agent) pairs): pair_kernel<.,1> runs BESIDE pair_kernel<.,0> (disjoint reservoirs)
+    // on this stream -- under a stream capture a parallel branch of the graph; at those sizes each launch is one
+    // warp's latency chain
     cudaStream_t pair_stream = nullptr;
     cudaEvent_t pair_fork = nullptr, pair_join = nullptr;
     int ev_threads = 128;              // event kernel: independent warps
@@ -351,33 +352,35 @@ static cudaError_t set_smem(const void* fn, size_t block_bytes, int threads, int
 
 static int launch_cfg(mlb_env* h) {
     const mlb_config& c = h->cfg;
-    const int A = c.num_agents;
-    const int SP = 32 * lanes_r(c.servers_per_agent);
+    const int A = c.num_agents, Sa = c.servers_per_agent;
+    const int SP = 32 * lanes_r(Sa);
     const bool alias = c.policy == MLB_POLICY_ALIAS;
-    if (getenv("MLB_HOST_CHUNKS")) h->host_chunks = atoi(getenv("MLB_HOST_CHUNKS"));
     h->ev_threads = 128;
     h->ev_smem = (size_t)(h->ev_threads / 32) * event_warp_smem_bytes(SP, alias);
-    h->epb = A == 1 ? (getenv("MLB_EPB") ? atoi(getenv("MLB_EPB")) : 4) : (A == 2 ? 2 : 1);
+    h->epb = A == 1 ? 4 : (A == 2 ? 2 : 1);
     h->ft_threads = 32 * A * h->epb;
     h->ft_smem = (size_t)(h->ft_threads / 32) * feature_warp_smem_bytes(SP) + (size_t)h->epb * 2 * h->d.S * 4;
     if (h->ft_threads > 1024) return fail(h, MLB_EINVAL, "num_agents > 32 not supported");
     if (h->ft_smem > 227 * 1024 || h->ev_smem > 227 * 1024)
         return fail(h, MLB_EINVAL, "configuration needs %zu B of shared memory per block (> 227 KB)",
                     h->ft_smem > h->ev_smem ? h->ft_smem : h->ev_smem);
-    cudaError_t e = set_smem(event_fn(c.policy, c.servers_per_agent, c.rng_mode), h->ev_smem, h->ev_threads, 4 * MLB_EV_MINBLOCKS);
-    if (e == cudaSuccess) e = set_smem(feature_fn(c.servers_per_agent, h->ft_threads <= 128 && !getenv("MLB_FT_BIG")), h->ft_smem, h->ft_threads, h->ft_threads <= 128 ? 48 : 32);
-    h->use_pair = h->d.KP == 128 && h->d.K == 128 && c.feature_cache == 1 && !getenv("MLB_NO_PAIR");
+    h->ev_fn = event_fn(c.policy, Sa, c.rng_mode);
+    h->ft_fn = feature_fn(Sa, h->ft_threads <= 128);
+    cudaError_t e = set_smem(h->ev_fn, h->ev_smem, h->ev_threads, 4 * EV_MIN_BLOCKS);
+    if (e == cudaSuccess) e = set_smem(h->ft_fn, h->ft_smem, h->ft_threads, h->ft_threads <= 128 ? 48 : 32);
+    h->use_pair = h->d.KP == 128 && c.feature_cache == 1;
     h->d.use_pair = h->use_pair ? 1 : 0;
     h->d.pair_wpe = 1;
-    h->pair_wpe_small = getenv("MLB_PAIR_WPE1") ? 1 : 4;    // A/B knob: 1 = never deal a list out to a block
-    if (h->use_pair && !h->pair_stream && !getenv("MLB_PAIR_SERIAL")) {
-        e = cudaStreamCreateWithFlags(&h->pair_stream, cudaStreamNonBlocking);
+    h->pr_smem = (size_t)4 * pair_warp_smem_bytes(SP);
+    if (h->use_pair) {
+        h->pr_fn[0] = pair_fn(Sa, 0);
+        h->pr_fn[1] = pair_fn(Sa, 1);
+        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->pair_stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pair_fork, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pair_join, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = set_smem(h->pr_fn[0], h->pr_smem, 128, 32);
+        if (e == cudaSuccess) e = set_smem(h->pr_fn[1], h->pr_smem, 128, 32);
     }
-    h->pr_smem = (size_t)4 * pair_warp_smem_bytes(SP);
-    if (e == cudaSuccess && h->use_pair) e = set_smem(pair_fn(c.servers_per_agent, 0), h->pr_smem, 128, 32);
-    if (e == cudaSuccess && h->use_pair) e = set_smem(pair_fn(c.servers_per_agent, 1), h->pr_smem, 128, 32);
     if (e != cudaSuccess) return fail(h, MLB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     return MLB_OK;
 }
@@ -893,22 +896,22 @@ static int launch_step(mlb_env* h, const void* dact, int e0, int e1, cudaStream_
     const int wpb = h->ev_threads / 32;
     const int ev_blocks = (int)(((int64_t)(e1 - e0) * dv.A + wpb - 1) / wpb);
     if (pe) CK(h, cudaEventRecord(pe[0], st));
-    CK(h, cudaLaunchKernel(event_fn(dv.policy, dv.Sa, dv.rng_mode), dim3(ev_blocks), dim3(h->ev_threads), ev_args, h->ev_smem, st));
+    CK(h, cudaLaunchKernel(h->ev_fn, dim3(ev_blocks), dim3(h->ev_threads), ev_args, h->ev_smem, st));
     if (pe) CK(h, cudaEventRecord(pe[1], st));
     void* ft_args[] = {&dv};
     if (h->use_pair) {
         const int64_t pairs = (int64_t)(e1 - e0) * dv.A;
-        dv.pair_wpe = pairs <= 8192 ? h->pair_wpe_small : 1;
+        dv.pair_wpe = pairs <= 8192 ? 4 : 1;
         const int pr_blocks = (int)(dv.pair_wpe == 4 ? pairs : (pairs + 3) / 4);
-        const bool beside = dv.pair_wpe == 4 && h->pair_stream != nullptr;
+        const bool beside = dv.pair_wpe == 4;
         cudaStream_t st1 = st;
         if (beside) {
             CK(h, cudaEventRecord(h->pair_fork, st));
             CK(h, cudaStreamWaitEvent(h->pair_stream, h->pair_fork, 0));
             st1 = h->pair_stream;
         }
-        CK(h, cudaLaunchKernel(pair_fn(dv.Sa, 0), dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st));
-        CK(h, cudaLaunchKernel(pair_fn(dv.Sa, 1), dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st1));
+        CK(h, cudaLaunchKernel(h->pr_fn[0], dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st));
+        CK(h, cudaLaunchKernel(h->pr_fn[1], dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st1));
         if (beside) {
             CK(h, cudaEventRecord(h->pair_join, h->pair_stream));
             CK(h, cudaStreamWaitEvent(st, h->pair_join, 0));
@@ -917,7 +920,7 @@ static int launch_step(mlb_env* h, const void* dact, int e0, int e1, cudaStream_
     }
     if (pe) CK(h, cudaEventRecord(pe[2], st));
     const int ft_blocks = (e1 - e0 + h->epb - 1) / h->epb;
-    CK(h, cudaLaunchKernel(feature_fn(dv.Sa, h->ft_threads <= 128 && !getenv("MLB_FT_BIG")), dim3(ft_blocks), dim3(h->ft_threads), ft_args, h->ft_smem, st));
+    CK(h, cudaLaunchKernel(h->ft_fn, dim3(ft_blocks), dim3(h->ft_threads), ft_args, h->ft_smem, st));
     if (pe) CK(h, cudaEventRecord(pe[3], st));
     h->launches += 2;
     return MLB_OK;

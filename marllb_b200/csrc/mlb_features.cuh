@@ -86,39 +86,6 @@ __device__ __forceinline__ void bitonic_sort_kv(float (&k)[EPL], float (&p)[EPL]
     bitonic_merge_levels<EPL, 2>(k, p, lane);
 }
 
-// blocked read of EPL consecutive floats per lane from shared memory
-template <int EPL>
-__device__ __forceinline__ void load_smem_block(const float* base, int lane, float (&x)[EPL]) {
-    if constexpr (EPL == 4) {
-        const float4 q = *reinterpret_cast<const float4*>(base + lane * 4);
-        x[0] = q.x; x[1] = q.y; x[2] = q.z; x[3] = q.w;
-    } else if constexpr (EPL == 2) {
-        const float2 q = *reinterpret_cast<const float2*>(base + lane * 2);
-        x[0] = q.x; x[1] = q.y;
-    } else {
-        x[0] = base[lane];
-    }
-}
-
-// element `slot` (warp-uniform) of an array spread EPL-per-lane.  Written as a select tree
-// on the sub-index bits: a sequential `if (sub == r) c = x[r]` chain makes nvcc materialise
-// x[] as a dynamically indexed local-memory array.
-template <int EPL, typename T>
-__device__ __forceinline__ T slot_fetch(const T (&x)[EPL], int slot) {
-    T c;
-    if constexpr (EPL == 4) {
-        const int sub = slot & 3;
-        const T lo = (sub & 1) ? x[1] : x[0];
-        const T hi = (sub & 1) ? x[3] : x[2];
-        c = (sub & 2) ? hi : lo;
-    } else if constexpr (EPL == 2) {
-        c = (slot & 1) ? x[1] : x[0];
-    } else {
-        c = x[0];
-    }
-    return __shfl_sync(MLB_FULL, c, slot / EPL);
-}
-
 template <int EPL>
 __device__ __forceinline__ void load_slots(const float* __restrict__ base, int lane, float (&x)[EPL]) {
     if constexpr (EPL == 4) {
@@ -207,109 +174,6 @@ __device__ __forceinline__ void ranks_full_sort(const float (&v)[EPL], int n, in
     const uint32_t packed = ranks_full_sort_packed<EPL>(sv, n, sc.vw);
 #pragma unroll
     for (int r = 0; r < EPL; r++) rk[r] = (packed >> (8 * r)) & 255u;
-}
-
-// ---------------------------------------------------------------------------
-// Incremental rank maintenance for a FULL reservoir (all 32*EPL slots valid) in which
-// Algorithm R replaced a few slots.  v[] already holds the new values, rk[] the ranks of
-// the previous contents.  Any order of equal values is a valid sorted order, and the stored
-// ranks may hold tied values in ANY order (the bitonic sort does not order ties), so the
-// update must not assume one: a new value is inserted AFTER every present element that
-// equals it -- "before" = (v_i <= x), "after" = (v_i > x), which is consistent with whatever
-// order the ties already have.  (Ranking ties by slot index instead, as this code first did,
-// produced duplicate ranks when a third equal value met a tied pair that a re-sort had left in
-// non-slot order; float32 durations taken as differences of timestamps are quantised, so such
-// triple ties do occur at scale: tools/determinism_probe.py, tests/test_gpu_ties.py.)
-//
-// One replaced slot c (the common case): remove its old rank, count the elements below
-// the new value, shift the ones above.  ~45 instructions.
-template <int EPL>
-__device__ __forceinline__ void rank_replace_one(const float (&v)[EPL], int (&rk)[EPL], int c, int lane) {
-    const int s0 = lane * EPL;
-    const float x = slot_fetch<EPL>(v, c);
-    const int r_old = slot_fetch<EPL>(rk, c);
-    bool before[EPL];
-    int cnt = 0;
-#pragma unroll
-    for (int r = 0; r < EPL; r++) {
-        before[r] = v[r] < x || (v[r] == x && s0 + r != c);  // v_i <= x for every other slot; false for i == c
-        cnt += before[r] ? 1 : 0;
-    }
-    const int r_new = __reduce_add_sync(MLB_FULL, cnt);
-#pragma unroll
-    for (int r = 0; r < EPL; r++) {
-        const int nr = rk[r] - (rk[r] > r_old ? 1 : 0) + (before[r] ? 0 : 1);
-        rk[r] = (s0 + r == c) ? r_new : nr;
-    }
-}
-
-// The same on the four ranks of a lane packed one per byte (full reservoir: every rank < 128),
-// with SWAR arithmetic for the shifts.  Returns the updated packed ranks.  ~45 instructions.
-__device__ __forceinline__ uint32_t rank_replace_one_packed(const float (&v)[4], uint32_t rkp, int c, int lane) {
-    const int sub = c & 3, lc = c >> 2;
-    const float xs = slot_fetch<4>(v, c);
-    const float x = xs + 0.0f;  // -0 -> +0, so that the integer successor below is the next float up
-    const uint32_t r_old = (__shfl_sync(MLB_FULL, rkp, lc) >> (8 * sub)) & 255u;
-    // v_i <= x  <=>  v_i < nextup(x) for every slot but c itself (which holds x and must not count)
-    const uint32_t xb = __float_as_uint(x);
-    const float xup = __uint_as_float((xb >> 31) ? xb - 1u : xb + 1u);
-    const int dl = c - lane * 4;  // slot r == dl of this lane is c
-    uint32_t bef = 0;
-#pragma unroll
-    for (int r = 0; r < 4; r++) {
-        const float xr = r == dl ? x : xup;
-        bef |= v[r] < xr ? (1u << (8 * r)) : 0u;
-    }
-    const uint32_t r_new = (uint32_t)__reduce_add_sync(MLB_FULL, __popc(bef));
-    // ranks above the removed one move down (bytes <= 127, so the borrow never crosses a byte),
-    // ranks at or above the inserted one move up
-    const uint32_t gt = (((rkp | 0x80808080u) - (r_old + 1u) * 0x01010101u) >> 7) & 0x01010101u;
-    rkp = rkp - gt + (bef ^ 0x01010101u);
-    if (lane == lc) rkp = (rkp & ~(255u << (8 * sub))) | (r_new << (8 * sub));
-    return rkp;
-}
-
-// General form (`list` = up to three 7-bit slot ids; slots >= n_old are appended, not
-// replaced; absent slots carry rank -1): first every old rank is taken out, then the new
-// values are inserted one at a time among the elements present so far.  Each sub-step leaves
-// a valid ranking of the present set.
-template <int EPL>
-__device__ __forceinline__ void rank_replace_few(const float (&v)[EPL], int (&rk)[EPL], uint32_t list, int nchg,
-                                                 int n_old, int lane) {
-    const int s0 = lane * EPL;
-#pragma unroll
-    for (int r = 0; r < EPL; r++) rk[r] = s0 + r < n_old ? rk[r] : -1;
-#pragma unroll 1
-    for (int k = 0; k < nchg; k++) {
-        const int c = (list >> (7 * k)) & 127;
-        if (c >= n_old) continue;  // appended slot: nothing to remove
-        const int r_old = slot_fetch<EPL>(rk, c);
-#pragma unroll
-        for (int r = 0; r < EPL; r++) {
-            rk[r] -= rk[r] > r_old ? 1 : 0;
-            rk[r] = (s0 + r == c) ? -1 : rk[r];
-        }
-    }
-#pragma unroll 1
-    for (int k = 0; k < nchg; k++) {
-        const int c = (list >> (7 * k)) & 127;
-        const float x = slot_fetch<EPL>(v, c);
-        bool after[EPL];
-        int cnt = 0;
-#pragma unroll
-        for (int r = 0; r < EPL; r++) {
-            const bool present = rk[r] >= 0;
-            const bool before = v[r] <= x;            // slot c itself is not present yet
-            after[r] = present && !before;
-            cnt += (present && before) ? 1 : 0;
-        }
-        const int r_new = __reduce_add_sync(MLB_FULL, cnt);
-#pragma unroll
-        for (int r = 0; r < EPL; r++) {
-            rk[r] += after[r] ? 1 : 0;
-            rk[r] = (s0 + r == c) ? r_new : rk[r];
-        }
-    }
 }
 
 // Cold paths of the weighted percentile, taken when the float32 cumulative weights come
@@ -414,11 +278,8 @@ __device__ __forceinline__ float fast_sqrt(float x) {
 // The five features given slot-ordered values/timestamps and valid ranks.
 // FULL: all 32*EPL slots are valid (n == 32*EPL), which makes n and everything derived from
 // it (p90 positions, interpolation weight, 1/n) compile-time constants.
-// DEFER: when the float32 weighted-percentile decision is not trusted, return false without
-// resolving it (the caller re-evaluates that reservoir on its cold path) instead of calling the
-// float64 tiers here, so that a hot loop contains no calls.
-template <int EPL, bool FULL, bool DEFER = false>
-__device__ __forceinline__ bool features_ranked(const float (&v)[EPL], const float (&t)[EPL],
+template <int EPL, bool FULL>
+__device__ __forceinline__ void features_ranked(const float (&v)[EPL], const float (&t)[EPL],
                                                 const int (&rk)[EPL], int n_, float now, double decay,
                                                 float log2_decay, const WarpScratch& sc, float (&out)[5]) {
     const int lane = lane_id();
@@ -483,10 +344,6 @@ __device__ __forceinline__ bool features_ranked(const float (&v)[EPL], const flo
     const uint32_t dmin_bits = __reduce_min_sync(MLB_FULL, __float_as_uint(dmin));
     if (__uint_as_float(dmin_bits) < MLB_WP_MARGIN * W) {
         // ---- not trusted: redo the decision in the reference's float64 arithmetic
-        if constexpr (DEFER) {
-            __syncwarp();  // scratch is reused by the next reservoir
-            return false;
-        }
         SlotVals<EPL> tv;
         uint32_t packed = 0;
 #pragma unroll
@@ -515,7 +372,6 @@ __device__ __forceinline__ bool features_ranked(const float (&v)[EPL], const flo
     out[2] = sd;
     out[3] = mean_decay;
     out[4] = p90_decay;
-    return true;
 }
 
 // Ranks from scratch, then the features: the stateless form (reservoir_features_kernel) and
@@ -575,7 +431,21 @@ __device__ __forceinline__ T pick8(const T (&x)[8], int sub) {
     return (sub & 4) ? hi : lo;
 }
 
-// rank_replace_one_packed on 8 slots per lane (ranks packed in two words)
+// Incremental rank maintenance for a reservoir in which Algorithm R replaced a few slots
+// (rank_replace_one_h16, rank_update_h16).  v[] already holds the new values, rkp[] the ranks of
+// the previous contents.  Any order of equal values is a valid sorted order, and the stored
+// ranks may hold tied values in ANY order (the bitonic sort does not order ties), so the
+// update must not assume one: a new value is inserted AFTER every present element that
+// equals it -- "before" = (v_i <= x), "after" = (v_i > x), which is consistent with whatever
+// order the ties already have.  (Ranking ties by slot index instead, as this code first did,
+// produced duplicate ranks when a third equal value met a tied pair that a re-sort had left in
+// non-slot order; float32 durations taken as differences of timestamps are quantised, so such
+// triple ties do occur at scale: tools/determinism_probe.py, tests/test_gpu_ties.py.)
+//
+// One replaced slot c of a FULL reservoir (the common case), ranks packed one per byte in two words: take out c's old
+// rank, count the elements below the new value x and shift the others with SWAR arithmetic.  v_i <= x is tested as
+// v_i < nextup(x) for every slot but c itself (which holds x and must not count); ranks above the removed one move
+// down (bytes <= 127, so the borrow never crosses a byte), ranks at or above the inserted one move up.
 __device__ __forceinline__ void rank_replace_one_h16(const float (&v)[8], uint32_t (&rkp)[2], int c, int hl,
                                                      int half) {
     const int sub = c & 7, lc = c >> 3;
@@ -602,8 +472,9 @@ __device__ __forceinline__ void rank_replace_one_h16(const float (&v)[8], uint32
     }
 }
 
-// features_ranked<4, true, DEFER> on 8 slots per lane; vw = this half's 128-entry scratch.
-// Returns false when the float32 weighted-percentile decision is not trusted (caller defers).
+// features_ranked<4, true> on 8 slots per lane; vw = this half's 128-entry scratch.
+// Returns false when the float32 weighted-percentile decision is not trusted (the caller hands the reservoir to
+// warp_features_ranked_exact) instead of calling the float64 tiers, so that the hot loop contains no calls.
 __device__ __forceinline__ bool features_full_h16(const float (&v)[8], const float (&t)[8], const uint32_t (&rkp)[2],
                                                   float log2_decay, float2* vw, int hl, int half,
                                                   float (&out)[5]) {
@@ -733,7 +604,8 @@ __device__ __forceinline__ void rank_update_h16(const float (&v)[8], uint32_t (&
     }
 }
 
-// features_ranked<4, false, DEFER> on 8 slots per lane: n valid slots (1..128), possibly different in the two halves
+// features_ranked<4, false> on 8 slots per lane, returning false like features_full_h16: n valid slots (1..128),
+// possibly different in the two halves
 __device__ __forceinline__ bool features_any_h16(const float (&v)[8], const float (&t)[8], const uint32_t (&rkp)[2],
                                                  int n, float log2_decay, float2* vw, int hl, int half,
                                                  float (&out)[5]) {
@@ -850,34 +722,8 @@ static __device__ __noinline__ float warp_features_ranked_exact(const float* __r
     load_slots<4>(vals, lane, v);
     load_slots<4>(tss, lane, t);
     load_ranks<4>(ranks, lane, rk);
-    features_ranked<4, false, false>(v, t, rk, n, now, decay, log2_decay, sc, f);
+    features_ranked<4, false>(v, t, rk, n, now, decay, log2_decay, sc, f);
     return feature_of_lane(f, lane);
-}
-
-// Steady state of the env step: a reservoir of 65..128 valid slots whose ranks live in global
-// memory next to it and in which Algorithm R wrote `nchg` <= 3 slots (7-bit ids in `list`;
-// slots >= n_old are appends of the fill phase) since those ranks were stored.
-// v, t: this lane's four slots; rkp: their stored ranks, one per byte; rank_out = &ranks[4 * lane].
-// Returns false if the weighted-percentile decision was not trusted (the caller then
-// re-evaluates the reservoir with warp_features_sorted); all lanes hold the same f[].
-__device__ __forceinline__ bool warp_features_incremental(const float (&v)[4], const float (&t)[4], uint32_t rkp,
-                                                          uint32_t* __restrict__ rank_out, int n, int n_old,
-                                                          uint32_t list, int nchg, float now, double decay,
-                                                          float log2_decay, const WarpScratch& sc, float (&f)[5]) {
-    const int lane = lane_id();
-    int rk[4];
-    if (n_old == 128 && nchg == 1) {
-        rkp = rank_replace_one_packed(v, rkp, (int)(list & 127u), lane);
-    } else {
-        rk[0] = rkp & 255; rk[1] = (rkp >> 8) & 255; rk[2] = (rkp >> 16) & 255; rk[3] = rkp >> 24;
-        rank_replace_few<4>(v, rk, list, nchg, n_old, lane);
-        rkp = (uint32_t)(rk[0] & 255) | ((uint32_t)(rk[1] & 255) << 8) | ((uint32_t)(rk[2] & 255) << 16) |
-              ((uint32_t)rk[3] << 24);
-    }
-    *rank_out = rkp;
-    rk[0] = rkp & 255; rk[1] = (rkp >> 8) & 255; rk[2] = (rkp >> 16) & 255; rk[3] = rkp >> 24;
-    if (n == 128) return features_ranked<4, true, true>(v, t, rk, 128, now, decay, log2_decay, sc, f);
-    return features_ranked<4, false, true>(v, t, rk, n, now, decay, log2_decay, sc, f);
 }
 
 }  // namespace mlb

@@ -39,9 +39,6 @@ constexpr int DRAIN_KB = 2;         // k-blocks accumulated in tensor memory bef
 constexpr int WORKER_WARPS = 8;
 constexpr int SPLIT_THREADS = 32 * WORKER_WARPS;   // 256
 constexpr int THREADS = 64 + SPLIT_THREADS;        // + TMA warp + MMA warp
-#ifndef MLB_TC_STORE_HI
-#define MLB_TC_STORE_HI 0   // 0: rely on the tensor core ignoring the low 13 mantissa bits of its inputs (measured: bit-identical results)
-#endif
 
 struct TcParams {
     float* C;
@@ -203,10 +200,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
                 l.y = __float_as_uint(__uint_as_float(v.y) - __uint_as_float(h.y)) & 0xffffe000u;
                 l.z = __float_as_uint(__uint_as_float(v.z) - __uint_as_float(h.z)) & 0xffffe000u;
                 l.w = __float_as_uint(__uint_as_float(v.w) - __uint_as_float(h.w)) & 0xffffe000u;
-#if MLB_TC_STORE_HI
-                hi[i] = h;
-#endif
-                lo[i] = l;
+                lo[i] = l;   // hi[i] keeps the raw value: the MMA ignores its low 13 mantissa bits (measured: bit-identical)
             };
 #pragma unroll
             for (int i = 0; i < (TILE_M * TILE_K / 4) / SPLIT_THREADS; i++) split(a_hi, a_lo, t + i * SPLIT_THREADS);

@@ -993,18 +993,12 @@ int mlb_gemm(const float* A, int64_t a_bs, int64_t a_rs, int64_t a_cs, const flo
              void* stream) {
     if (!A || !B || !C || M < 0 || N < 0 || K < 0 || batch < 1) return MLB_EINVAL;
     if (M == 0 || N == 0) return MLB_OK;
-    // single products big enough to fill tensor-core tiles go to the tcgen05 kernel (csrc/mlb_gemm_tc.cu); MLB_GEMM_TC_MIN
-    // (multiply-adds, default 2^21; 0 disables) is an A/B knob
-    {
-        static const int64_t tc_min = [] {
-            const char* e = getenv("MLB_GEMM_TC_MIN");
-            return e ? (int64_t)atoll(e) : (int64_t)1 << 21;
-        }();
-        if (batch == 1 && tc_min > 0 && (int64_t)M * N * K >= tc_min &&
-            mlb_gemm_tc_supported(A, a_rs, a_cs, B, b_rs, b_cs, C, ldc, M, N, K)) {
-            const int rc = mlb_gemm_tc(A, a_rs, a_cs, B, b_rs, b_cs, C, ldc, bias, M, N, K, beta, act, stream);
-            if (rc != MLB_ESTATE && rc != MLB_ENOMEM) return rc;   // those two: nothing was launched, use the FFMA kernel
-        }
+    // single products big enough to fill tensor-core tiles (>= 2^21 multiply-adds) go to the tcgen05 kernel
+    // (csrc/mlb_gemm_tc.cu)
+    if (batch == 1 && (int64_t)M * N * K >= ((int64_t)1 << 21) &&
+        mlb_gemm_tc_supported(A, a_rs, a_cs, B, b_rs, b_cs, C, ldc, M, N, K)) {
+        const int rc = mlb_gemm_tc(A, a_rs, a_cs, B, b_rs, b_cs, C, ldc, bias, M, N, K, beta, act, stream);
+        if (rc != MLB_ESTATE && rc != MLB_ENOMEM) return rc;   // those two: nothing was launched, use the FFMA kernel
     }
     if (batch == 1 && K >= 1) {
         cudaStream_t st = (cudaStream_t)stream;

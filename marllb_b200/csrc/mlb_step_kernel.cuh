@@ -57,12 +57,9 @@ __host__ __device__ inline size_t event_warp_smem_bytes(int SP, bool alias) {
     return (size_t)NF * SP * 4 + (alias ? (size_t)SP * (8 + 4 + 8 + 4) : 0);
 }
 
-// ---- feature kernel: per-warp shared memory = dirty list | rank-order scratch | staging buffer
-// staging buffer: values[128] | timestamps[128] | ranks[128 bytes] of the NEXT reservoir,
-// filled by cp.async while the current one is being evaluated
-#define MLB_STAGE_BYTES 1152
+// ---- feature kernel: per-warp shared memory = dirty list | rank-order scratch
 __host__ __device__ inline size_t feature_warp_smem_bytes(int SP) {
-    return (size_t)2 * SP * 8 + MLB_SCRATCH_BYTES + MLB_STAGE_BYTES;
+    return (size_t)2 * SP * 8 + MLB_SCRATCH_BYTES;
 }
 
 // Assignment score of one server as an order-preserving uint.
@@ -314,11 +311,9 @@ __device__ __noinline__ double reward_staged(int metric, const T* rv, const uint
 
 // ---------------------------------------------------------------------------
 // event_kernel: R = servers per lane (Sa <= 32*R), SP = 32*R.  Warps are independent.
-#ifndef MLB_EV_MINBLOCKS
-#define MLB_EV_MINBLOCKS 10
-#endif
+constexpr int EV_MIN_BLOCKS = 10;   // resident blocks per SM the registers are budgeted for (40 warps)
 template <int POLICY, int R, int RNG>
-__global__ void __launch_bounds__(128, MLB_EV_MINBLOCKS)
+__global__ void __launch_bounds__(128, EV_MIN_BLOCKS)
 event_kernel(const __grid_constant__ DevState d, const void* __restrict__ action) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int SP = 32 * R;
@@ -556,17 +551,22 @@ event_kernel(const __grid_constant__ DevState d, const void* __restrict__ action
 }
 
 // ---------------------------------------------------------------------------
-// pair_kernel: the steady state of the statistics -- FULL 128-slot reservoirs in which Algorithm R replaced
-// exactly one slot -- two reservoirs per warp instruction (one per half-warp, 8 slots per lane; see
-// mlb_features.cuh).  One warp per (env, agent), warps independent.  A separate kernel so that its loop
-// (~420 instructions per pair) has the instruction cache to itself: inside feature_kernel the two hot
-// paths evicted each other (ncu: 29 % of the stalls were instruction fetches).
+// pair_kernel: the incremental statistics of every cached reservoir with a 128-slot stride (K = 97..128) whose
+// stored ranks are valid and in which Algorithm R wrote 1..3 slots -- two reservoirs per warp instruction (one per
+// half-warp, 8 slots per lane; see mlb_features.cuh).  One warp per (env, agent), warps independent.  A separate
+// kernel so that its loop (~420 instructions per pair) has the instruction cache to itself: inside feature_kernel
+// the two hot paths evicted each other (ncu: 29 % of the stalls were instruction fetches).
+//
+// Shared memory per warp: dirty list | two rank-order scratches | two staging buffers.  A staging buffer holds
+// values[128] | timestamps[128] | ranks[128 bytes] of one reservoir of the NEXT pair, filled by cp.async while the
+// current pair is being evaluated.
+#define MLB_STAGE_BYTES 1152
 __host__ __device__ inline size_t pair_warp_smem_bytes(int SP) {
     return (size_t)2 * SP * 8 + 2 * MLB_SCRATCH_BYTES + 2 * MLB_STAGE_BYTES;
 }
 
 // CLS 0: full reservoirs with ONE replaced slot (constants folded, one-slot SWAR update);
-// CLS 1: every other incrementally updatable reservoir (2-3 written slots, fill-phase appends, any n).
+// CLS 1: every other incrementally updatable reservoir (2-3 written slots, fill-phase appends, K < 128).
 template <int R, int CLS>
 __global__ void __launch_bounds__(128, 8)
 pair_kernel(const __grid_constant__ DevState d) {
@@ -603,7 +603,7 @@ pair_kernel(const __grid_constant__ DevState d) {
                 cnt = __ldg(d.res_count + c);
             }
             const uint32_t nchg = chg_count(chg);
-            const uint32_t n = cnt < 128u ? cnt : 128u;
+            const uint32_t n = cnt < (uint32_t)d.K ? cnt : (uint32_t)d.K;
             const bool one = nchg == 1 && chg_nold(chg) == 128 && n == 128;
             // n_old == 255: pair_kernel<.,0> could not settle this one and handed it to feature_kernel.  On small launches
             // the two pair kernels run side by side, so <.,1> may or may not see that mark yet -- either way the entry is
@@ -624,7 +624,9 @@ pair_kernel(const __grid_constant__ DevState d) {
     uint32_t off0 = (uint32_t)(sbase * 2 * 32) + (uint32_t)lane;
     uint32_t obs0 = (uint32_t)(sbase * MLB_OBS_COLS) + 1u;
     uint32_t chg0 = (uint32_t)((size_t)e * 2 * S + seed0);
-    asm volatile("" : "+r"(off0), "+r"(obs0), "+r"(chg0));   // keep them in registers (see feature_kernel)
+    // opaque to the optimiser: otherwise they are re-derived from (env, agent) with 64-bit multiplies inside the loop
+    // instead of living in three registers
+    asm volatile("" : "+r"(off0), "+r"(obs0), "+r"(chg0));
     const uint32_t stage_s = (uint32_t)__cvta_generic_to_shared(stage) + lane * 16;
     const int half = lane >> 4, hl = lane & 15;
     float2* const vw_half = vw + half * 128;
@@ -708,12 +710,11 @@ feature_kernel(const __grid_constant__ DevState d) {
     const int e = d.e0 + blockIdx.x * epb + env_in_blk;
     if (e >= d.e1) return;  // whole env (all its warps) leaves together
 
-    // ---- shared memory: [per warp: dirty list | scratch | stage] ... [per env: reward staging]
+    // ---- shared memory: [per warp: dirty list | scratch] ... [per env: reward staging]
     const size_t wbytes = feature_warp_smem_bytes(SP);
     unsigned char* wbase = smem_raw + (size_t)warp * wbytes;
     uint2* dlist = reinterpret_cast<uint2*>(wbase);
     const WarpScratch scratch{reinterpret_cast<float2*>(wbase + (size_t)2 * SP * 8)};
-    unsigned char* stage = wbase + (size_t)2 * SP * 8 + MLB_SCRATCH_BYTES;
     float* rv = reinterpret_cast<float*>(smem_raw + (size_t)nwarps * wbytes) + (size_t)env_in_blk * 2 * S;
     uint32_t* ra = reinterpret_cast<uint32_t*>(rv + S);
 
@@ -728,16 +729,12 @@ feature_kernel(const __grid_constant__ DevState d) {
 
     // ---------------- phase B: statistics of touched reservoirs --------------
     // The dirty (server, metric) pairs are first compacted into a list, every lane describing
-    // its own servers: entry = { changed-slot word, id | n << 9 | incremental << 17 }.
-    // The loop over that list is then a plain counted loop in which the NEXT reservoir
-    // (values, timestamps, ranks: 1152 B) is copied into the warp's staging buffer with
-    // cp.async while the current one is evaluated from registers.
+    // its own servers: entry = { changed-slot word, id | n << 9 | redo << 18 }.
     const bool all = d.feature_cache == 0;  // mode 0: recompute every reservoir
     const int KP = d.KP;
-    const bool staged = KP == 128 && d.feature_cache == 1;
-    // "Fast" entries (full reservoir, exactly one replaced slot: the steady state) were already evaluated by
-    // pair_kernel, two per warp instruction; an entry it could not settle comes back with its change count
-    // saturated (-> re-sorted here).  This kernel takes everything else.
+    // Entries with valid stored ranks and 1..3 written slots were already evaluated by pair_kernel; an entry it
+    // could not settle comes back with n_old = 255 ("redo": ranks valid, float64 decision needed).  This kernel
+    // takes everything else.
     int nd = 0;
 #pragma unroll
     for (int r = 0; r < R; r++) {
@@ -752,80 +749,20 @@ feature_kernel(const __grid_constant__ DevState d) {
             }
             const uint32_t nchg = chg_count(chg);
             const uint32_t n = cnt < (uint32_t)d.K ? cnt : (uint32_t)d.K;
-            const bool redo = chg_nold(chg) == 255u;   // pair_kernel: ranks valid, float64 decision needed
-            const bool inc = staged && !redo && chg_nold(chg) > 0 && nchg >= 1 && nchg <= 3;
-            const bool fast = d.use_pair && inc;       // pair_kernel<.,0> / <.,1> took these
+            const bool redo = chg_nold(chg) == 255u;
+            const bool fast = d.use_pair && !redo && chg_nold(chg) > 0 && nchg >= 1 && nchg <= 3;
             const bool take = j < Sa && (all || nchg > 0) && !fast;
             const unsigned bal = __ballot_sync(MLB_FULL, take);
             if (take)
                 dlist[nd + __popc(bal & ((1u << lane) - 1u))] =
-                    make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9) | ((inc ? 1u : 0u) << 17) | ((redo ? 1u : 0u) << 18));
+                    make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9) | ((redo ? 1u : 0u) << 18));
             nd += __popc(bal);
         }
     }
     __syncwarp();
     float* const warp_obs = obs + 1;
-    int ncold = 0;
-    if (staged) {
-        // 32-bit offsets from the array bases (mlb_create checks that they fit): one number
-        // addresses this lane's four slots of a reservoir in all three arrays
-        //   values / timestamps: float4 index;  ranks: uint32 index
-        const float4* const val4 = reinterpret_cast<const float4*>(d.res_val);
-        const float4* const ts4 = reinterpret_cast<const float4*>(d.res_ts);
-        uint32_t* const rank4 = reinterpret_cast<uint32_t*>(d.res_rank);
-        uint32_t off0 = (uint32_t)(sbase * 2 * 32) + (uint32_t)lane;
-        uint32_t obs0 = (uint32_t)(sbase * MLB_OBS_COLS) + 1u;      // column 1 of this warp's first server
-        // opaque to the optimiser: otherwise both are re-derived from (env, agent) with 64-bit multiplies
-        // inside the loop instead of living in two registers
-        asm volatile("" : "+r"(off0), "+r"(obs0));
-        const uint32_t stage_s = (uint32_t)__cvta_generic_to_shared(stage) + lane * 16;
-        const float4* stage_v = reinterpret_cast<const float4*>(stage) + lane;
-        auto stage_in = [&](uint32_t id) {
-            const uint32_t off = off0 + id * 32u;
-            cp_async16(stage_s, val4 + off);
-            cp_async16(stage_s + 512, ts4 + off);
-            cp_async4(stage_s + 1024 - lane * 12, rank4 + off);
-            cp_async_commit();
-        };
-        if (nd > 0) stage_in(dlist[0].y & 511u);
 #pragma unroll 1
-        for (int i = 0; i < nd; i++) {
-            const uint2 ent = dlist[i];
-            cp_async_wait_all();
-            __syncwarp();
-            const float4 qv = stage_v[0];
-            const float4 qt = stage_v[32];
-            const uint32_t rkp = reinterpret_cast<const uint32_t*>(stage_v - lane + 64)[lane];
-            __syncwarp();
-            if (i + 1 < nd) stage_in(dlist[i + 1].y & 511u);
-            // anything that is not "a few replaced slots, trusted float32 decision" is deferred to
-            // the cold loop below (entries re-packed at the front of the list): no calls in here
-            bool ok = false;
-            if ((ent.y >> 17) & 1u) {
-                const uint32_t id = ent.y & 511u;
-                const float v[4] = {qv.x, qv.y, qv.z, qv.w};
-                const float t[4] = {qt.x, qt.y, qt.z, qt.w};
-                float f[5];
-                ok = warp_features_incremental(v, t, rkp, rank4 + (off0 + id * 32u), (int)((ent.y >> 9) & 255u),
-                                               (int)chg_nold(ent.x), ent.x, (int)chg_count(ent.x), t1, d.decay,
-                                               d.log2_decay, scratch, f);
-                if (ok && lane == 0) {
-                    float* o = d.obs + (obs0 + (id >> 1) * MLB_OBS_COLS + (id & 1u) * 5u);
-#pragma unroll
-                    for (int q = 0; q < 5; q++) o[q] = f[q];
-                }
-            }
-            if (!ok) {
-                if (lane == 0) dlist[ncold] = ent;
-                ncold++;
-            }
-        }
-        __syncwarp();
-    } else {
-        ncold = nd;
-    }
-#pragma unroll 1
-    for (int i = 0; i < ncold; i++) {
+    for (int i = 0; i < nd; i++) {
         const uint2 ent = dlist[i];
         const uint32_t id = ent.y & 511u;
         const int n = (int)((ent.y >> 9) & 255u);

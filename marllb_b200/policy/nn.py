@@ -279,10 +279,6 @@ def linear_backward(P, wname, bname, x, dy, need_dx=True):
     return ops.matmul_nn(dy, P.p[wname]) if need_dx else None
 
 
-import os as _os
-FUSED_GRU_SEQ = _os.environ.get("MLB_FUSED_GRU_SEQ", "1") != "0"   # A/B knob: 0 = the step-by-step launches
-
-
 class GRUCellSeq:
     """nn.GRU(in, H, batch_first=True) run step by step (agent_network.py:41,76-78; networks.py:60,97)."""
 
@@ -303,7 +299,7 @@ class GRUCellSeq:
         T, B, In = xs.shape
         H = h0.shape[-1]
         gi_all = ops.linear(xs.reshape(T * B, In), P[k + "weight_ih_l0"], P[k + "bias_ih_l0"]).reshape(T, B, 3 * H)
-        if FUSED_GRU_SEQ and ops.gru_seq_supported(H):
+        if ops.gru_seq_supported(H):
             # the whole time loop in one launch (csrc/mlb_policy.cu gru_seq_fwd_kernel)
             hs, hprev, ghs, gates = ops.gru_seq_forward(gi_all.contiguous(), P[k + "weight_hh_l0"], P[k + "bias_hh_l0"],
                                                         h0.contiguous())
@@ -327,7 +323,7 @@ class GRUCellSeq:
         P, k = self.P, self.k
         xs, hprev, ghs, gates = tape
         T, B, H = dhs.shape
-        if FUSED_GRU_SEQ and ops.gru_seq_supported(H):
+        if ops.gru_seq_supported(H):
             dgi_all, dgh_all, dh_next = ops.gru_seq_backward(dhs.contiguous(), gates, hprev, ghs, P.p[k + "weight_hh_l0"])
             return self._seq_param_grads(dgi_all, dgh_all, xs, hprev, need_dx, dh_next)
         dgi_all = torch.empty_like(gates)

@@ -136,8 +136,7 @@ def _chk(t):
     return t
 
 
-import os as _os
-TC_MIN_M = int(_os.environ.get("MLB_TC_MIN_M", "512"))   # below this the tile launch overhead beats the FFMA kernel's
+TC_MIN_M = 512   # below this the tile launch overhead beats the FFMA kernel's
 
 
 def linear_tc(x, W, b=None, act=ACT_NONE, out=None):

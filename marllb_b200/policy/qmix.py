@@ -14,7 +14,6 @@ block.  `strict_reference=False` gathers each agent's own Q.
 from __future__ import annotations
 
 import contextlib
-import os
 import random
 from collections import deque
 from pathlib import Path
@@ -378,9 +377,6 @@ class QMIXAgent:
         self.episode_buffer = EpisodeBuffer(capacity=buffer_capacity, num_agents=num_agents)
         self.graph_updates = False      # True: replay the device part of update() as a CUDA graph
         self._graphs = {}
-        # inside a stream capture the per-agent chains of update() (online and target forwards, backwards) are issued on
-        # several streams = parallel branches of the graph (MLB_QMIX_BRANCHES=0: one stream); eager updates use one stream
-        self.parallel_branches = os.environ.get("MLB_QMIX_BRANCHES", "1") != "0"
         self._aux = None
         self.total_updates = 0
         self.training_stats = {'loss': [], 'q_tot': [], 'target_q_tot': []}
@@ -472,8 +468,7 @@ class QMIXAgent:
             torch.cuda.current_stream(self.device).wait_stream(side)
             torch.cuda.synchronize(self.device)
             self._restore(snap)
-            if self.parallel_branches:
-                ops.reserve_workspace_slots(4)      # split-K workspaces of the side lanes (nothing can be allocated in a capture)
+            ops.reserve_workspace_slots(4)          # split-K workspaces of the side lanes (nothing can be allocated in a capture)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
                 out = self._update_device(*static)
@@ -506,7 +501,7 @@ class QMIXAgent:
         # each other and each keeps only a handful of SMs busy (the GRU time loop of B = 32 episodes is 8 thread blocks):
         # while the update is being captured they go to separate streams ("lanes"), i.e. parallel branches of the graph.
         cur = torch.cuda.current_stream(dev)
-        multi = self.parallel_branches and torch.cuda.is_current_stream_capturing()
+        multi = torch.cuda.is_current_stream_capturing()
         if multi and self._aux is None:
             self._aux = [torch.cuda.Stream(device=dev) for _ in range(3)]
         lanes = [None] + self._aux if multi else [None]

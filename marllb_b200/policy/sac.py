@@ -13,7 +13,6 @@ passed (parity tests pass the reference's draws).
 from __future__ import annotations
 
 import contextlib
-import os
 import random
 from collections import deque
 from pathlib import Path
@@ -320,11 +319,6 @@ class SAC_GRU_Agent:
             self.alpha = torch.tensor([alpha], dtype=torch.float32, device=self.device)
             self.target_entropy = None
         self.replay_buffer = ReplayBuffer(capacity=buffer_size)
-        # update_parameters on several streams (Q2's passes beside Q1's, parameter gradients beside the input-gradient
-        # chain, the actor's forward beside the critic steps).  "graph" (default): only while the update is being
-        # captured into a CUDA graph, where the streams become parallel branches -- launched eagerly the update is bound
-        # by Python launch overhead and the stream switches only add to it; "always"; "off".  MLB_SAC_TWIN = 0 / 1 / 2.
-        self.twin_streams = {"0": "off", "1": "graph", "2": "always"}.get(os.environ.get("MLB_SAC_TWIN", "1"), "graph")
         self._twin = None
         self.total_steps = 0
         self.training_stats = {'q1_loss': [], 'q2_loss': [], 'policy_loss': [], 'alpha_loss': [], 'alpha': []}
@@ -377,9 +371,10 @@ class SAC_GRU_Agent:
             # on the caller's stream.  At batch 256 each network is a dependent chain of small kernels that leave most
             # of the 148 SMs idle, so the two chains overlap almost entirely; inside a CUDA graph they become parallel
             # branches.  Arithmetic and step order are unchanged (sac_agent.py:201-231: Q1 step, Q2 step, actor, alpha).
+            # Only while the update is being captured: launched eagerly it is bound by Python launch overhead, and the
+            # stream switches would only add to it.
             cur = torch.cuda.current_stream(self.device)
-            multi = self.twin_streams == "always" or (self.twin_streams == "graph" and torch.cuda.is_current_stream_capturing())
-            twin = self._twin_stream() if multi else None
+            twin = self._twin_stream() if torch.cuda.is_current_stream_capturing() else None
 
             def fork():
                 if twin is not None:
@@ -473,7 +468,7 @@ class SAC_GRU_Agent:
             if a_loss is not None:
                 losses['alpha'] = losses['alpha'] + conv(a_loss)
             self.total_steps += 1
-            if twin is None and self.twin_streams == "graph":
+            if twin is None:
                 ops.reserve_workspace_slots(5)      # a later capture of this update finds its side streams' split-K workspaces
         for k in losses:
             losses[k] = losses[k] / updates

@@ -9,8 +9,8 @@ value met a tied pair in the other order.  tools/determinism_probe.py found it a
 size (7 envs of 131072 within 2148 steps).  Here arrival times and work sit on a 1/32 s grid, so EVERY duration is a
 multiple of 1/32 s and every reservoir is mostly ties; the observations must equal the C oracle's (which sorts from
 scratch every step, like the reference: reservoir.py:105-196) over a long episode, through every statistics path:
-pair kernels (default), the 4-slots-per-lane incremental path of feature_kernel (MLB_NO_PAIR=1) and full re-sorts
-(feature_cache=False).
+the pair kernels at K = 128, the pair kernels at K = 112 (a 128-slot stride with full reservoirs below 128 slots, whose
+replacements take the general incremental update) and full re-sorts (feature_cache=False).
 """
 import os
 import sys
@@ -37,12 +37,10 @@ def _grid_streams(rng, E, Sa, rate, horizon):
     return out
 
 
-@pytest.mark.parametrize("mode", ["pair", "no_pair", "resort"])
-def test_tied_values_through_every_statistics_path(mode, monkeypatch):
+@pytest.mark.parametrize("mode", ["pair", "pair_k112", "resort"])
+def test_tied_values_through_every_statistics_path(mode):
     from marllb_b200 import VecLoadBalanceEnv
-    if mode == "no_pair":
-        monkeypatch.setenv("MLB_NO_PAIR", "1")
-    E, Sa, steps, rate, K = 6, 8, 900, 48.0, 128
+    E, Sa, steps, rate, K = 6, 8, 900, 48.0, 112 if mode == "pair_k112" else 128
     rng = np.random.RandomState(4242)
     speeds = np.where(np.arange(Sa) % 2 == 0, 1.0, 2.0).astype(np.float32)
     streams = _grid_streams(rng, E, Sa, rate, steps * 0.25 + 0.5)

@@ -1,6 +1,6 @@
 """Quick device-side timing of the env step at the bench's c5 slice, without per-kernel profiling events:
     python tools/quick_ms.py [--envs N] [--burnin B] [--steps K]
-Environment variables of the library (MLB_OVERLAP, MLB_AUX_HIGH, ...) apply.  Prints ms per step."""
+MARLLB_B200_LIB=marllb_b200/_variants/NAME.so times a variant built by tools/build_variant.sh.  Prints ms per step."""
 import argparse
 import os
 import sys
@@ -45,7 +45,7 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     env.check_status()
-    tag = " ".join(f"{k}={v}" for k, v in sorted(os.environ.items()) if k.startswith("MLB_"))
+    tag = os.environ.get("MARLLB_B200_LIB", "in-tree library")
     print(f"[{tag}] {e0.elapsed_time(e1) / a.steps:.3f} ms per step, checksum {float(env.obs.sum(dtype=torch.float64)):.6e}")
 
 
