@@ -153,6 +153,7 @@ __global__ void reset_kernel(const DevState d, const uint8_t* __restrict__ mask)
     for (int i = tid; i < 2 * S; i += nt) {
         d.res_count[(size_t)e * 2 * S + i] = 0;
         d.res_cursor[(size_t)e * 2 * S + i] = 0;
+        d.res_tie[(size_t)e * 2 * S + i] = 0;
     }
     const size_t rn = (size_t)S * 2 * d.KP;
     float4* v4 = reinterpret_cast<float4*>(d.res_val + sb * 2 * d.KP);
@@ -218,7 +219,8 @@ __global__ void gen_poisson_kernel(float* __restrict__ time, float* __restrict__
 // ------------------------------------------------------------------ changed-rows compaction
 // One thread per (env, server) row of envs [e0, e1): writes the row's n_flow_on into the dense 16-bit column and,
 // when Algorithm R wrote a slot of either reservoir of the row this step (res_chg, written by event_kernel for
-// every reservoir), appends {row index, the 11 observation floats} to this chunk's record list.
+// every reservoir) or feature_kernel re-evaluated one of them as an exact tie (res_tie), appends {row index, the 11
+// observation floats} to this chunk's record list.
 __global__ void compact_rows_kernel(const DevState d, uint32_t* __restrict__ rec, uint16_t* __restrict__ col,
                                     uint32_t* __restrict__ cnt) {
     const int S = d.S;
@@ -230,7 +232,8 @@ __global__ void compact_rows_kernel(const DevState d, uint32_t* __restrict__ rec
     bool changed = false;
     if (in) {
         const uint32_t c0 = d.res_chg[((size_t)e * 2 + 0) * S + sv], c1 = d.res_chg[((size_t)e * 2 + 1) * S + sv];
-        changed = d.feature_cache != 1 || ((c0 >> 21) & 7u) != 0u || ((c1 >> 21) & 7u) != 0u;
+        changed = d.feature_cache != 1 || ((c0 >> 21) & 7u) != 0u || ((c1 >> 21) & 7u) != 0u ||
+                  d.res_tie[((size_t)e * 2 + 0) * S + sv] != 0 || d.res_tie[((size_t)e * 2 + 1) * S + sv] != 0;
         col[row] = (uint16_t)d.n_on[row];
     }
     const unsigned bal = __ballot_sync(MLB_FULL, changed);
@@ -554,6 +557,7 @@ int mlb_create(const mlb_config* cfg, mlb_env** out) {
     CKC(dalloc(h, &d.res_cursor, ES * 2));
     CKC(dalloc(h, &d.res_rank, ES * 2 * d.KP));
     CKC(dalloc(h, &d.res_chg, ES * 2));
+    CKC(dalloc(h, &d.res_tie, ES * 2));
     CKC(dalloc(h, &d.ring, ES * d.Q));
     CKC(dalloc(h, &d.obs, ES * MLB_OBS_COLS));
     CKC(dalloc(h, &d.reward, (size_t)d.E));

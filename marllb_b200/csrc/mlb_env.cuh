@@ -38,6 +38,7 @@ struct DevState {
     uint32_t* res_cursor;
     uint8_t* res_rank;     // [E][S][2][KP] rank of each slot's value (order statistics cache)
     uint32_t* res_chg;     // [E][2][S] slots written this step (event kernel -> feature kernel)
+    uint8_t* res_tie;      // [E][2][S] 1: the last p90_decay decision was an exact tie (feature kernel re-evaluates it)
     // ---- FIFO rings [E][S][Q]
     float2* ring;          // (arrival time, finish time) of every in-system flow
     // ---- outputs

@@ -214,16 +214,95 @@ static __device__ __noinline__ int weighted_index_scan_f64(const float2* st, int
     return __reduce_add_sync(MLB_FULL, below);
 }
 
+// Correctly rounded decay^y for tier 3.  Tier 3 runs when a cumulative weight sits within 1e-9 of the cutoff,
+// in practice an exact tie in real arithmetic (e.g. ten samples of one timestamp, the cutoff on the ninth).  There
+// the reference's decision hangs on the last bit of each weight, which the host's pow rounds correctly for all but a
+// few arguments while CUDA's pow may be 2 ulp off.  exp(y * ln(decay)) in double-double arithmetic (~2^-95 relative
+// error) rounds correctly.
+// Explicitly rounded operations: a contraction into fma would break the error-free transforms.
+struct DD {
+    double hi, lo;
+};
+__device__ __forceinline__ double dd_rn_add(double a, double b) {
+    return __dadd_rn(a, b);
+}
+__device__ __forceinline__ double dd_rn_mul(double a, double b) {
+    return __dmul_rn(a, b);
+}
+__device__ __forceinline__ double dd_rn_fma(double a, double b, double c) {
+    return __fma_rn(a, b, c);
+}
+__device__ __forceinline__ DD dd_two_sum(double a, double b) {
+    const double s = dd_rn_add(a, b), bb = dd_rn_add(s, -a);
+    return {s, dd_rn_add(dd_rn_add(a, -dd_rn_add(s, -bb)), dd_rn_add(b, -bb))};
+}
+__device__ __forceinline__ DD dd_quick_two_sum(double a, double b) {   // |a| >= |b|
+    const double s = dd_rn_add(a, b);
+    return {s, dd_rn_add(b, -dd_rn_add(s, -a))};
+}
+__device__ __forceinline__ DD dd_add(DD a, DD b) {
+    DD s = dd_two_sum(a.hi, b.hi);
+    const DD t = dd_two_sum(a.lo, b.lo);
+    s = dd_quick_two_sum(s.hi, dd_rn_add(s.lo, t.hi));
+    return dd_quick_two_sum(s.hi, dd_rn_add(s.lo, t.lo));
+}
+__device__ __forceinline__ DD dd_mul(DD a, DD b) {
+    const double p = dd_rn_mul(a.hi, b.hi);
+    const double e = dd_rn_fma(a.lo, b.hi, dd_rn_fma(a.hi, b.lo, dd_rn_fma(a.hi, b.hi, -p)));
+    return dd_quick_two_sum(p, e);
+}
+__device__ __forceinline__ DD dd_mul_d(DD a, double b) {
+    const double p = dd_rn_mul(a.hi, b);
+    return dd_quick_two_sum(p, dd_rn_fma(a.lo, b, dd_rn_fma(a.hi, b, -p)));
+}
+// e^z = 2^k e^r, e^r = (e^(r/1024))^1024: Taylor series of e^s - 1 to s^9 (|s| < 3.4e-4), then ten squarings of
+// 1 + x as x <- 2x + x^2.  Returns the double-double value, |z| < 700.
+__device__ inline DD dd_exp(DD z) {
+    const DD ln2 = {0x1.62e42fefa39efp-1, 0x1.abc9e3b39803fp-56};
+    const double k = rint(dd_rn_mul(z.hi, 0x1.71547652b82fep0));
+    DD r = dd_add(z, dd_mul_d(ln2, -k));
+    r.hi = dd_rn_mul(r.hi, 0x1p-10);
+    r.lo = dd_rn_mul(r.lo, 0x1p-10);
+    DD p = {0.0, 0.0};
+    double fact = 362880.0;                       // 9!
+    for (int m = 9; m >= 1; m--) {                // p <- p * s + 1/m!
+        const double c = 1.0 / fact;
+        p = dd_add(dd_mul(p, r), DD{c, dd_rn_fma(-c, fact, 1.0) / fact});
+        fact /= m;
+    }
+    DD x = dd_mul(p, r);
+    for (int i = 0; i < 10; i++) x = dd_add(DD{dd_rn_mul(x.hi, 2.0), dd_rn_mul(x.lo, 2.0)}, dd_mul(x, x));
+    const DD e = dd_add(DD{1.0, 0.0}, x);
+    return {ldexp(e.hi, (int)k), ldexp(e.lo, (int)k)};
+}
+// ln(decay) as a double-double: one Newton step on log(decay).
+__device__ inline DD dd_log(double d) {
+    const double l0 = log(d);
+    const DD e = dd_exp(DD{l0, 0.0});
+    const DD num = dd_add(DD{d, 0.0}, DD{-e.hi, -e.lo});
+    return dd_two_sum(l0, dd_rn_add(num.hi, num.lo) / e.hi);
+}
+// decay^y rounded to nearest, given ln_decay = dd_log(decay).
+__device__ inline double pow_cr(double decay, DD ln_decay, double y) {
+    if (y == 0.0 || decay == 1.0) return 1.0;
+    const DD z = dd_mul_d(ln_decay, y);
+    // beyond e^-700 (a weight older than ~6600 s at decay 0.9) the result leaves the normal range, where ldexp would
+    // round a second time: CUDA's pow decides there, so a tie among weights that small may go the other way
+    if (!(fabs(z.hi) < 700.0)) return pow(decay, y);
+    return dd_exp(z).hi;
+}
+
 // Tier 3: the reference's own arithmetic (reservoir.py:148-149,181-196): w = pow(decay, now - t)
-// and a strictly sequential cumsum in value order.  Returns the searchsorted-left index of
-// 0.9 * cumsum[-1] (n if none).
+// (correctly rounded, as the host's pow) and a strictly sequential cumsum in value order.  Returns the
+// searchsorted-left index of 0.9 * cumsum[-1] (n if none).
 static __device__ __noinline__ int weighted_index_f64(const float2* st, int n, float now, double decay) {
     const int lane = lane_id();
+    const DD ln_decay = dd_log(decay);
     double w[4];
 #pragma unroll
     for (int k = 0; k < 4; k++) {
         const int pos = k * 32 + lane;
-        w[k] = pos < n ? pow(decay, (double)now - (double)st[pos].y) : 0.0;
+        w[k] = pos < n ? pow_cr(decay, ln_decay, (double)now - (double)st[pos].y) : 0.0;
     }
     double c = 0.0;
 #pragma unroll 1
@@ -248,7 +327,8 @@ static __device__ __noinline__ int weighted_index_f64(const float2* st, int n, f
     return idx;
 }
 
-// Both float64 tiers; out of line so the steady-state loop stays small.
+// Both float64 tiers; out of line so the steady-state loop stays small.  Returns the index, plus 0x100 when tier 2
+// found an exact tie and tier 3 decided it.
 template <int EPL>
 __device__ __noinline__ int weighted_index_exact(SlotVals<EPL> t, uint32_t rk_packed, int n, float tmax, float now,
                                                  double decay, float2* vw) {
@@ -260,7 +340,7 @@ __device__ __noinline__ int weighted_index_exact(SlotVals<EPL> t, uint32_t rk_pa
     __syncwarp();
     bool ambiguous;
     int idx = weighted_index_scan_f64(vw, n, tmax, decay, &ambiguous);
-    if (ambiguous) idx = weighted_index_f64(vw, n, now, decay);
+    if (ambiguous) idx = weighted_index_f64(vw, n, now, decay) | 0x100;
     return idx;
 }
 
@@ -277,14 +357,17 @@ __device__ __forceinline__ float fast_sqrt(float x) {
 
 // The five features given slot-ordered values/timestamps and valid ranks.
 // FULL: all 32*EPL slots are valid (n == 32*EPL), which makes n and everything derived from
-// it (p90 positions, interpolation weight, 1/n) compile-time constants.
+// it (p90 positions, interpolation weight, 1/n) compile-time constants.  `tie` is set when the
+// p90_decay index sits on an exact tie (decided by tier 3).
 template <int EPL, bool FULL>
 __device__ __forceinline__ void features_ranked(const float (&v)[EPL], const float (&t)[EPL],
                                                 const int (&rk)[EPL], int n_, float now, double decay,
-                                                float log2_decay, const WarpScratch& sc, float (&out)[5]) {
+                                                float log2_decay, const WarpScratch& sc, float (&out)[5],
+                                                bool& tie) {
     const int lane = lane_id();
     const int s0 = lane * EPL;
     const int n = FULL ? 32 * EPL : n_;
+    tie = false;
     // ---- mean (np.mean on float32: reservoir.py:143), newest timestamp
     float s = 0.f, tmax = -MLB_INF;
 #pragma unroll
@@ -352,6 +435,8 @@ __device__ __forceinline__ void features_ranked(const float (&v)[EPL], const flo
             packed |= (uint32_t)(rk[r] & 255) << (8 * r);
         }
         idx = weighted_index_exact<EPL>(tv, packed, n, tmax, now, decay, sc.vw);
+        tie = idx >= 0x100;
+        idx &= 0xff;
     }
     idx = idx > n - 1 ? n - 1 : idx;  // reservoir.py:193-194
     // ---- p90 = np.percentile(values, 90): float32 'linear' rule of numpy >= 2
@@ -380,7 +465,8 @@ __device__ __forceinline__ void features_ranked(const float (&v)[EPL], const flo
 template <int EPL>
 __device__ __forceinline__ void features_sorted_epl(const float* __restrict__ vals, const float* __restrict__ tss,
                                                     uint8_t* __restrict__ ranks, int n, float now, double decay,
-                                                    float log2_decay, const WarpScratch& sc, float (&out)[5]) {
+                                                    float log2_decay, const WarpScratch& sc, float (&out)[5],
+                                                    bool& tie) {
     const int lane = lane_id();
     float v[EPL], t[EPL];
     int rk[EPL];
@@ -389,9 +475,9 @@ __device__ __forceinline__ void features_sorted_epl(const float* __restrict__ va
     ranks_full_sort<EPL>(v, n, rk, sc);
     if (ranks) store_ranks<EPL>(ranks, lane, rk);
     if (n == 32 * EPL)
-        features_ranked<EPL, true>(v, t, rk, n, now, decay, log2_decay, sc, out);
+        features_ranked<EPL, true>(v, t, rk, n, now, decay, log2_decay, sc, out, tie);
     else
-        features_ranked<EPL, false>(v, t, rk, n, now, decay, log2_decay, sc, out);
+        features_ranked<EPL, false>(v, t, rk, n, now, decay, log2_decay, sc, out, tie);
 }
 
 // ---------------------------------------------------------------------------
@@ -682,36 +768,37 @@ __device__ __forceinline__ bool features_any_h16(const float (&v)[8], const floa
     return ok;
 }
 
-// lane q < 5 keeps feature q (the lane that stores it)
-__device__ __forceinline__ float feature_of_lane(const float (&f)[5], int lane) {
+// lane q < 5 keeps feature q (the lane that stores it); lane 5 gets 1 when p90_decay sits on an exact tie
+__device__ __forceinline__ float feature_of_lane(const float (&f)[5], bool tie, int lane) {
     float mine = f[0];
 #pragma unroll
     for (int q = 1; q < 5; q++) mine = lane == q ? f[q] : mine;
-    return mine;
+    return lane == 5 ? (tie ? 1.f : 0.f) : mine;
 }
 
-// Returns feature `lane` in lanes 0..4.
+// Returns feature `lane` in lanes 0..4, the exact-tie flag in lane 5.
 static __device__ __noinline__ float warp_features_sorted(const float* __restrict__ vals, const float* __restrict__ tss,
                                                           uint8_t* __restrict__ ranks, int n, float now, double decay,
                                                           float log2_decay, float2* scratch) {
     const WarpScratch sc{scratch};
     float f[5];
+    bool tie = false;
     if (n <= 0) {  // reservoir.py:127-134
 #pragma unroll
         for (int q = 0; q < 5; q++) f[q] = 0.f;
     } else if (n <= 32) {
-        features_sorted_epl<1>(vals, tss, ranks, n, now, decay, log2_decay, sc, f);
+        features_sorted_epl<1>(vals, tss, ranks, n, now, decay, log2_decay, sc, f, tie);
     } else if (n <= 64) {
-        features_sorted_epl<2>(vals, tss, ranks, n, now, decay, log2_decay, sc, f);
+        features_sorted_epl<2>(vals, tss, ranks, n, now, decay, log2_decay, sc, f, tie);
     } else {
-        features_sorted_epl<4>(vals, tss, ranks, n, now, decay, log2_decay, sc, f);
+        features_sorted_epl<4>(vals, tss, ranks, n, now, decay, log2_decay, sc, f, tie);
     }
-    return feature_of_lane(f, lane_id());
+    return feature_of_lane(f, tie, lane_id());
 }
 
 // Ranks in global memory are valid (an incremental kernel updated and stored them) but its float32
 // weighted-percentile decision was not trusted: evaluate from the stored ranks with the float64 tiers,
-// no re-sort.  128-slot stride.  Returns feature `lane` in lanes 0..4.
+// no re-sort.  128-slot stride.  Returns feature `lane` in lanes 0..4, the exact-tie flag in lane 5.
 static __device__ __noinline__ float warp_features_ranked_exact(const float* __restrict__ vals, const float* __restrict__ tss,
                                                                 const uint8_t* __restrict__ ranks, int n, float now,
                                                                 double decay, float log2_decay, float2* scratch) {
@@ -722,8 +809,9 @@ static __device__ __noinline__ float warp_features_ranked_exact(const float* __r
     load_slots<4>(vals, lane, v);
     load_slots<4>(tss, lane, t);
     load_ranks<4>(ranks, lane, rk);
-    features_ranked<4, false>(v, t, rk, n, now, decay, log2_decay, sc, f);
-    return feature_of_lane(f, lane);
+    bool tie;
+    features_ranked<4, false>(v, t, rk, n, now, decay, log2_decay, sc, f, tie);
+    return feature_of_lane(f, tie, lane);
 }
 
 }  // namespace mlb

@@ -734,28 +734,31 @@ feature_kernel(const __grid_constant__ DevState d) {
     const int KP = d.KP;
     // Entries with valid stored ranks and 1..3 written slots were already evaluated by pair_kernel; an entry it
     // could not settle comes back with n_old = 255 ("redo": ranks valid, float64 decision needed).  This kernel
-    // takes everything else.
+    // takes everything else, and also untouched reservoirs whose p90_decay sat on an exact tie: the reference
+    // decides such a tie anew every step, from weights rescaled to the new `now` whose last bits differ.
     int nd = 0;
 #pragma unroll
     for (int r = 0; r < R; r++) {
         const int j = lane + 32 * r;
 #pragma unroll
         for (int m = 0; m < 2; m++) {
-            uint32_t chg = 0, cnt = 0;
+            uint32_t chg = 0, cnt = 0, tie = 0;
+            const size_t c = ((size_t)e * 2 + m) * S + seed0 + j;
             if (j < Sa) {
-                const size_t c = ((size_t)e * 2 + m) * S + seed0 + j;
                 chg = __ldg(d.res_chg + c);
                 cnt = __ldg(d.res_count + c);
+                tie = d.res_tie[c];
             }
             const uint32_t nchg = chg_count(chg);
             const uint32_t n = cnt < (uint32_t)d.K ? cnt : (uint32_t)d.K;
             const bool redo = chg_nold(chg) == 255u;
             const bool fast = d.use_pair && !redo && chg_nold(chg) > 0 && nchg >= 1 && nchg <= 3;
-            const bool take = j < Sa && (all || nchg > 0) && !fast;
+            const bool take = j < Sa && (all || nchg > 0 || tie) && !fast;
+            if (fast && tie) d.res_tie[c] = 0;   // pair_kernel trusted its float32 decision: no longer a tie
             const unsigned bal = __ballot_sync(MLB_FULL, take);
             if (take)
                 dlist[nd + __popc(bal & ((1u << lane) - 1u))] =
-                    make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9) | ((redo ? 1u : 0u) << 18));
+                    make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9) | ((redo ? 1u : 0u) << 18) | (tie << 19));
             nd += __popc(bal);
         }
     }
@@ -775,6 +778,8 @@ feature_kernel(const __grid_constant__ DevState d) {
             mine = warp_features_sorted(res_val + rid, res_ts + rid, res_rank + rid, n, t1, d.decay,
                                         d.log2_decay, scratch.vw);
         if (lane < 5) warp_obs[(id >> 1) * MLB_OBS_COLS + (id & 1u) * 5u + lane] = mine;
+        const uint32_t tie = __shfl_sync(MLB_FULL, mine, 5) != 0.f ? 1u : 0u;
+        if (lane == 0 && tie != ((ent.y >> 19) & 1u)) d.res_tie[((size_t)e * 2 + (id & 1u)) * S + seed0 + (id >> 1)] = (uint8_t)tie;
     }
     __syncwarp();
 
