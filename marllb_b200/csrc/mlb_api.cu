@@ -51,11 +51,12 @@ struct mlb_env {
     size_t action_bytes = 0;
     uint8_t* d_mask = nullptr;
     size_t ev_smem = 0, ft_smem = 0, pr_smem = 0;   // dynamic shared memory of the event / feature / pair kernel
-    const void *ev_fn = nullptr, *ft_fn = nullptr, *pr_fn[2] = {nullptr, nullptr};   // kernel instantiations of this config
+    // kernel instantiations of this config; pr_fn[c] = pair_kernel<R, c>
+    const void *ev_fn = nullptr, *ft_fn = nullptr, *pr_fn[3] = {nullptr, nullptr, nullptr};
     bool use_pair = false;             // pair_kernel applies (128-slot reservoir stride, feature cache on)
-    // small launches (<= 8192 (env, agent) pairs): pair_kernel<.,1> runs BESIDE pair_kernel<.,0> (disjoint reservoirs)
-    // on this stream -- under a stream capture a parallel branch of the graph; at those sizes each launch is one
-    // warp's latency chain
+    // large launches (> 8192 (env, agent) pairs) run both classes in one pair_kernel<.,2>; small ones run
+    // pair_kernel<.,1> BESIDE pair_kernel<.,0> (disjoint reservoirs) on this stream -- under a stream capture a
+    // parallel branch of the graph; at those sizes each launch is one warp's latency chain
     cudaStream_t pair_stream = nullptr;
     cudaEvent_t pair_fork = nullptr, pair_join = nullptr;
     int ev_threads = 128;              // event kernel: independent warps
@@ -332,12 +333,13 @@ static const void* feature_fn(int Sa, bool small) {
     }
 }
 
-static const void* pair_fn(int Sa, int cls) {
+template <int CLS>
+static const void* pair_fn_c(int Sa) {
     switch (lanes_r(Sa)) {
-    case 1: return cls ? (const void*)pair_kernel<1, 1> : (const void*)pair_kernel<1, 0>;
-    case 2: return cls ? (const void*)pair_kernel<2, 1> : (const void*)pair_kernel<2, 0>;
-    case 4: return cls ? (const void*)pair_kernel<4, 1> : (const void*)pair_kernel<4, 0>;
-    default: return cls ? (const void*)pair_kernel<8, 1> : (const void*)pair_kernel<8, 0>;
+    case 1: return (const void*)pair_kernel<1, CLS>;
+    case 2: return (const void*)pair_kernel<2, CLS>;
+    case 4: return (const void*)pair_kernel<4, CLS>;
+    default: return (const void*)pair_kernel<8, CLS>;
     }
 }
 
@@ -376,13 +378,13 @@ static int launch_cfg(mlb_env* h) {
     h->d.pair_wpe = 1;
     h->pr_smem = (size_t)4 * pair_warp_smem_bytes(SP);
     if (h->use_pair) {
-        h->pr_fn[0] = pair_fn(Sa, 0);
-        h->pr_fn[1] = pair_fn(Sa, 1);
+        h->pr_fn[0] = pair_fn_c<0>(Sa);
+        h->pr_fn[1] = pair_fn_c<1>(Sa);
+        h->pr_fn[2] = pair_fn_c<2>(Sa);
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->pair_stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pair_fork, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pair_join, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = set_smem(h->pr_fn[0], h->pr_smem, 128, 32);
-        if (e == cudaSuccess) e = set_smem(h->pr_fn[1], h->pr_smem, 128, 32);
+        for (int k = 0; k < 3 && e == cudaSuccess; k++) e = set_smem(h->pr_fn[k], h->pr_smem, 128, 32);
     }
     if (e != cudaSuccess) return fail(h, MLB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     return MLB_OK;
@@ -905,22 +907,21 @@ static int launch_step(mlb_env* h, const void* dact, int e0, int e1, cudaStream_
     void* ft_args[] = {&dv};
     if (h->use_pair) {
         const int64_t pairs = (int64_t)(e1 - e0) * dv.A;
-        dv.pair_wpe = pairs <= 8192 ? 4 : 1;
-        const int pr_blocks = (int)(dv.pair_wpe == 4 ? pairs : (pairs + 3) / 4);
-        const bool beside = dv.pair_wpe == 4;
-        cudaStream_t st1 = st;
-        if (beside) {
+        if (pairs <= 8192) {
+            // four warps per (env, agent), both classes side by side
+            dv.pair_wpe = 4;
             CK(h, cudaEventRecord(h->pair_fork, st));
             CK(h, cudaStreamWaitEvent(h->pair_stream, h->pair_fork, 0));
-            st1 = h->pair_stream;
-        }
-        CK(h, cudaLaunchKernel(h->pr_fn[0], dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st));
-        CK(h, cudaLaunchKernel(h->pr_fn[1], dim3(pr_blocks), dim3(128), ft_args, h->pr_smem, st1));
-        if (beside) {
+            CK(h, cudaLaunchKernel(h->pr_fn[0], dim3((int)pairs), dim3(128), ft_args, h->pr_smem, st));
+            CK(h, cudaLaunchKernel(h->pr_fn[1], dim3((int)pairs), dim3(128), ft_args, h->pr_smem, h->pair_stream));
             CK(h, cudaEventRecord(h->pair_join, h->pair_stream));
             CK(h, cudaStreamWaitEvent(st, h->pair_join, 0));
+            h->launches += 2;
+        } else {
+            // one warp per (env, agent), both classes in one launch
+            CK(h, cudaLaunchKernel(h->pr_fn[2], dim3((int)((pairs + 3) / 4)), dim3(128), ft_args, h->pr_smem, st));
+            h->launches += 1;
         }
-        h->launches += 2;
     }
     if (pe) CK(h, cudaEventRecord(pe[2], st));
     const int ft_blocks = (e1 - e0 + h->epb - 1) / h->epb;

@@ -555,7 +555,9 @@ event_kernel(const __grid_constant__ DevState d, const void* __restrict__ action
 // stored ranks are valid and in which Algorithm R wrote 1..3 slots -- two reservoirs per warp instruction (one per
 // half-warp, 8 slots per lane; see mlb_features.cuh).  One warp per (env, agent), warps independent.  A separate
 // kernel so that its loop (~420 instructions per pair) has the instruction cache to itself: inside feature_kernel
-// the two hot paths evicted each other (ncu: 29 % of the stalls were instruction fetches).
+// the two hot paths evicted each other (ncu: 29 % of the stalls were instruction fetches).  The two classes below
+// share a kernel (CLS 2) on large launches: class 0 waits on DRAM, class 1 on issue slots, and only warps of one
+// launch share an SM once a grid of that size has taken every SM.
 //
 // Shared memory per warp: dirty list | two rank-order scratches | two staging buffers.  A staging buffer holds
 // values[128] | timestamps[128] | ranks[128 bytes] of one reservoir of the NEXT pair, filled by cp.async while the
@@ -566,18 +568,21 @@ __host__ __device__ inline size_t pair_warp_smem_bytes(int SP) {
 }
 
 // CLS 0: full reservoirs with ONE replaced slot (constants folded, one-slot SWAR update);
-// CLS 1: every other incrementally updatable reservoir (2-3 written slots, fill-phase appends, K < 128).
+// CLS 1: every other incrementally updatable reservoir (2-3 written slots, fill-phase appends, K < 128);
+// CLS 2: both classes in one launch (large launches): the class-0 pairs of a warp's list first, then its class-1 pairs,
+//        so that resident warps of the two classes -- one DRAM-bound, one issue-bound -- share each SM.
 template <int R, int CLS>
 __global__ void __launch_bounds__(128, 8)
 pair_kernel(const __grid_constant__ DevState d) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int SP = 32 * R;
+    constexpr bool kBoth = CLS == 2;
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int A = d.A, Sa = d.Sa, S = d.S;
     // Large launches: one warp per (env, agent).  Small ones (a few thousand envs: a fraction of a wave, where the time
     // is one warp's walk through its list) deal the list of one (env, agent) out to the four warps of a block.
-    const int wpe = d.pair_wpe;
+    const int wpe = kBoth ? 1 : d.pair_wpe;
     const int ea = d.e0 * A + (wpe == 1 ? blockIdx.x * (blockDim.x >> 5) + warp : (int)blockIdx.x);
     const int sub = wpe == 1 ? 0 : warp;
     if (ea >= d.e1 * A) return;
@@ -590,7 +595,9 @@ pair_kernel(const __grid_constant__ DevState d) {
     const size_t sbase = (size_t)e * S + (size_t)agent * Sa;
     const int seed0 = agent * Sa;
 
-    int nfast = 0;
+    // The warp's list: class-0 entries from the front of dlist; class-1 entries after them, or -- CLS 2, which learns
+    // the class-0 count only at the end of this one pass over the words -- from the back, in reverse order.
+    int n0 = 0, n1 = 0;
 #pragma unroll
     for (int r = 0; r < R; r++) {
         const int j = lane + 32 * r;
@@ -610,14 +617,34 @@ pair_kernel(const __grid_constant__ DevState d) {
             // not its own ("one" before the mark, "redo" after it).
             const bool redo = chg_nold(chg) == 255u;
             const bool inc = !redo && chg_nold(chg) > 0 && nchg >= 1 && nchg <= 3;
-            const bool fast = j < Sa && (CLS == 0 ? one : (inc && !one));
-            const unsigned bal = __ballot_sync(MLB_FULL, fast);
-            if (fast) dlist[nfast + __popc(bal & ((1u << lane) - 1u))] = make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9));
-            nfast += __popc(bal);
+            const uint2 entry = make_uint2(chg, (uint32_t)(j * 2 + m) | (n << 9));
+            const unsigned below = (1u << lane) - 1u;
+            if (CLS != 1) {
+                const bool fast = j < Sa && one;
+                const unsigned bal = __ballot_sync(MLB_FULL, fast);
+                if (fast) dlist[n0 + __popc(bal & below)] = entry;
+                n0 += __popc(bal);
+            }
+            if (CLS != 0) {
+                const bool fast = j < Sa && inc && !one;
+                const unsigned bal = __ballot_sync(MLB_FULL, fast);
+                const int k = n1 + __popc(bal & below);
+                if (fast) dlist[kBoth ? 2 * SP - 1 - k : k] = entry;
+                n1 += __popc(bal);
+            }
         }
     }
     __syncwarp();
-    if (nfast == 0) return;
+    // wpe 4: the four warps of a block build the same list, and a warp writes n_old = 255 marks (below) into words the
+    // others may not have read yet -- a list that lost an entry would skip one reservoir and update another twice
+    if (!kBoth && wpe != 1) __syncthreads();
+    // List positions [0, p0) are class 0, [p0, np) class 1.  p0 is n0 rounded up to a whole pair, so that no pair mixes
+    // the classes: an odd class-0 segment ends with half 1 idle, like the end of a list.
+    const int p0 = CLS == 1 ? 0 : (kBoth ? (n0 + 1) & ~1 : n0);
+    const int np = p0 + n1;
+    auto at = [&](int q) { return kBoth && q >= p0 ? 2 * SP - 1 - (q - p0) : q; };   // dlist index of position q
+    auto live = [&](int q) { return q < (kBoth && q < p0 ? n0 : np); };
+    if (np == 0) return;
     const float4* const val4 = reinterpret_cast<const float4*>(d.res_val);
     const float4* const ts4 = reinterpret_cast<const float4*>(d.res_ts);
     uint32_t* const rank4 = reinterpret_cast<uint32_t*>(d.res_rank);
@@ -638,14 +665,14 @@ pair_kernel(const __grid_constant__ DevState d) {
         cp_async4(dst + 1024 - lane * 12, rank4 + off);
     };
     const int i0 = 2 * sub, di = 2 * wpe;     // this warp takes the pairs i0, i0 + di, ...
-    if (i0 >= nfast) return;
-    stage_in(dlist[i0].y & 511u, 0);
-    if (i0 + 1 < nfast) stage_in(dlist[i0 + 1].y & 511u, 1);
+    if (i0 >= np) return;
+    stage_in(dlist[at(i0)].y & 511u, 0);
+    if (live(i0 + 1)) stage_in(dlist[at(i0 + 1)].y & 511u, 1);
     cp_async_commit();
 #pragma unroll 1
-    for (int i = i0; i < nfast; i += di) {
-        const bool valid = i + half < nfast;              // an odd list ends with half 1 idle
-        const uint2 ent = dlist[valid ? i + half : i];
+    for (int i = i0; i < np; i += di) {
+        const bool valid = live(i + half);                // an odd list ends with half 1 idle
+        const uint2 ent = dlist[at(valid ? i + half : i)];
         const uint32_t id = ent.y & 511u;
         cp_async_wait_all();
         __syncwarp();
@@ -654,9 +681,9 @@ pair_kernel(const __grid_constant__ DevState d) {
         const float4 t0 = reinterpret_cast<const float4*>(rec + 512)[hl * 2], t1q = reinterpret_cast<const float4*>(rec + 512)[hl * 2 + 1];
         const uint2 rq = reinterpret_cast<const uint2*>(rec + 1024)[hl];
         __syncwarp();
-        if (i + di < nfast) {
-            stage_in(dlist[i + di].y & 511u, 0);
-            if (i + di + 1 < nfast) stage_in(dlist[i + di + 1].y & 511u, 1);
+        if (i + di < np) {                                // CLS 2: runs on across the class boundary
+            stage_in(dlist[at(i + di)].y & 511u, 0);
+            if (live(i + di + 1)) stage_in(dlist[at(i + di + 1)].y & 511u, 1);
             cp_async_commit();
         }
         const float v[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
@@ -664,7 +691,7 @@ pair_kernel(const __grid_constant__ DevState d) {
         uint32_t rkp[2] = {valid ? rq.x : 0u, valid ? rq.y : 0u};   // idle half: every scatter position 0
         float f[5];
         bool ok;
-        if (CLS == 0) {
+        if (CLS == 0 || (kBoth && i < p0)) {
             rank_replace_one_h16(v, rkp, (int)(ent.x & 127u), hl, half);
             if (valid) reinterpret_cast<uint2*>(rank4 + (off0 - lane + id * 32u))[hl] = make_uint2(rkp[0], rkp[1]);
             if (!valid) { rkp[0] = 0u; rkp[1] = 0u; }

@@ -25,13 +25,13 @@ seq = [(r[0], r[kn].split('(')[0].strip(), float(r[mv].replace(',', ''))) for r 
 mlb = [x for x in seq if 'mlb::' in x[1]]
 agg = collections.OrderedDict()
 for _, n, tm in seq: agg.setdefault(n, []).append(tm)
-timed = mlb[4 * 259:4 * 279]
+timed = mlb[3 * 259:3 * 279]   # three launches per bench-size step
 per = collections.OrderedDict()
 for _, n, tm in timed: per.setdefault(n, []).append(tm)
 tot = sum(sum(v) for v in per.values())
 with open('profiles/r01_launches_four_kernel_step.csv', 'w') as fo:
     fo.write("# ncu --metrics gpu__time_duration.sum --clock-control none; python bench.py --steps 20 --warmup 3 --no-cpu --e2e-steps 2 (256 burn-in steps)\n")
-    fo.write("# per-launch times are cold-cache and serialised: shares matter, not absolutes. A step = event_kernel + pair_kernel<.,0> + pair_kernel<.,1> + feature_kernel.\n")
+    fo.write("# per-launch times are cold-cache and serialised: shares matter, not absolutes. A step = event_kernel + pair_kernel<.,2> (both statistics classes) + feature_kernel.\n")
     fo.write("# whole run (burn-in included: in the first steps after reset every touched reservoir is re-sorted by feature_kernel)\n")
     fo.write("kernel,launches,total_ms,mean_us\n")
     for k, v in agg.items(): fo.write(f"\"{k[:80]}\",{len(v)},{sum(v)/1e6:.3f},{sum(v)/len(v)/1e3:.1f}\n")
